@@ -2,6 +2,7 @@
 """bench.py — the hot path of BASELINE.json measured on B200(s).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config c2|c3|c4|c5] [--mesh soup|grid]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Default (`--config c2`, BASELINE.json configs[1]): a step is one pass of the batched closest-hit traversal
@@ -52,6 +53,7 @@ CONFIGS = {
 }
 AUTO_DIRECT_MAX_RANKS = 4         # --gather auto: per-record peer stores up to this many ranks, staged bulk copies beyond
 C4_CPU_ROW_STRIDE = 10           # the CPU arm of c4 traces every 10th image row (10M of the 100M rays)
+DUMP_MAX_RAYS = 1 << 20          # --dump-outputs: at most this many hit records (28 MB in f32, 40 MB in f64)
 
 
 def parse_args():
@@ -75,7 +77,14 @@ def parse_args():
                          "record — or NCCL all-gather")
     ap.add_argument("--sort-rays", action="store_true", help="BVH_SORT_RAYS: traverse the batch in the Morton order of the ray origins")
     ap.add_argument("--no-numa", action="store_true", help="N > 1: do not bind the rank to its GPU's NUMA node")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the hit records of the last timed step as DIR/<field>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs writes the outputs of the CUDA path")
+    return args
 
 
 def hbm_peak():
@@ -255,6 +264,21 @@ def bytes_per_ray(cfg, s_inner, s_tri):
     if cfg["dtype"] == "f64":
         return 64 + 32 + 128 * s_inner + 96 * s_tri
     return 32 + (4 if cfg["any_hit"] else 16) + 64 * s_inner + 48 * s_tri
+
+
+def dump_outputs(out_dir, hits, hit_dtype):
+    """Writes the hit records the timed path returned (all ranks' rays, in global ray order) as float arrays, so that
+    two builds run with the same arguments can be compared output for output: prim_id (float64; exact for every id, a
+    miss is the all-ones id), t, u, v (the config's precision) and ray_index (float64, the ray each record belongs to).
+    Batches larger than DUMP_MAX_RAYS are represented by a fixed, seeded sample of DUMP_MAX_RAYS rays."""
+    rec = hits.cpu().numpy().view(hit_dtype).reshape(-1)
+    n = rec.shape[0]
+    index = np.arange(n) if n <= DUMP_MAX_RAYS else np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_RAYS, replace=False))
+    rec = rec[index]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("prim_id", rec["prim_id"].astype(np.float64)), ("t", rec["t"]), ("u", rec["u"]), ("v", rec["v"]),
+                    ("ray_index", index.astype(np.float64))):
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -547,6 +571,8 @@ def main():
         ref_sums = sums.clone()
         dist.broadcast(ref_sums, src=0)
         assert torch.equal(sums, ref_sums), "ranks disagree on the gathered hit records"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, tracer.global_hits(), hit_dtype)
 
     # ---- e2e through the C ABI with pinned host buffers ----------------------------------------------
     e2e = None

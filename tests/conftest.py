@@ -22,14 +22,6 @@ def oracle():
 
 
 @pytest.fixture(scope="session")
-def ref():
-    from oracle.pyoracle import Ref, ref_available
-    if not ref_available():
-        pytest.skip("oracle/_ref/libbvh_ref.so not built (needs /root/reference at build time)")
-    return Ref()
-
-
-@pytest.fixture(scope="session")
 def emul():
     from tests.helpers import HostEmul
     return HostEmul()

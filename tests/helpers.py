@@ -1,5 +1,7 @@
 """Test helpers: the host emulation of the device code (tests/host_emul.cpp) and comparison utilities."""
 import ctypes as C
+import hashlib
+import json
 import os
 import subprocess
 
@@ -158,6 +160,43 @@ def assert_hits_equal(got, want, what=""):
         else:
             same = a.astype(np.uint64) == b.astype(np.uint64)
         assert same.all(), f"{what}: {name} differs at {np.nonzero(~same)[0][:8]} ({(~same).sum()} of {same.size})"
+
+
+def digest(a) -> str:
+    """SHA-256 of an array's dtype, shape and bytes (bytes objects count as uint8 arrays): equal digests mean
+    bit-identical arrays, so a stored digest pins an output of the reference as strictly as the output itself."""
+    a = np.ascontiguousarray(np.frombuffer(a, np.uint8) if isinstance(a, bytes) else a)
+    return hashlib.sha256(a.dtype.str.encode() + repr(a.shape).encode() + a.tobytes()).hexdigest()
+
+
+def ref_digests(key):
+    """Digests of the reference's outputs for one test case (tests/golden/make_ref_digests.py)."""
+    with open(os.path.join(ROOT, "tests", "golden", "ref_digests.json")) as f:
+        return json.load(f)[key]
+
+
+def tree_blob(index, prim_ids, boxes, dim):
+    """The reference's file format (bvh.h serialize) of the tree with the given topology over `boxes` ([n, 2*dim]: mins then
+    maxes): every node box is the exact union of the primitive boxes below it, as the reference's builders make them.
+    Index words and prim ids are 32-bit for float trees and 64-bit for double trees; children follow their parent."""
+    dtype = boxes.dtype
+    it = np.dtype(np.uint32 if dtype == np.float32 else np.uint64)
+    index = np.asarray(index, np.uint64)
+    prim_ids = np.asarray(prim_ids, np.int64)
+    lo, hi = boxes[:, :dim], boxes[:, dim:]
+    bounds = np.empty((index.shape[0], 2 * dim), dtype)
+    for i in range(index.shape[0] - 1, -1, -1):
+        first, count = int(index[i] >> np.uint64(4)), int(index[i] & np.uint64(15))
+        if count:
+            ids = prim_ids[first:first + count]
+            bounds[i, 0::2], bounds[i, 1::2] = lo[ids].min(axis=0), hi[ids].max(axis=0)
+        else:
+            assert first > i, "a child precedes its parent"
+            bounds[i, 0::2] = np.minimum(bounds[first, 0::2], bounds[first + 1, 0::2])
+            bounds[i, 1::2] = np.maximum(bounds[first, 1::2], bounds[first + 1, 1::2])
+    nodes = np.zeros(index.shape[0], [("bounds", dtype, 2 * dim), ("index", it)])
+    nodes["bounds"], nodes["index"] = bounds, index
+    return np.array([index.shape[0], prim_ids.shape[0]], it).tobytes() + nodes.tobytes() + prim_ids.astype(it).tobytes()
 
 
 def hits_tuple(hits):

@@ -52,3 +52,35 @@ def test_gather_form_follows_the_rank_count():
     assert bench.gather_candidates(8, "auto") == ["multicast_staged", "peer", "direct"]        # falls back when there is no multicast address
     for mode in ("multicast", "multicast_staged", "peer", "direct"):
         assert bench.gather_candidates(8, mode) == [mode]
+
+
+def test_dump_outputs_writes_a_fixed_sample_as_floats(tmp_path):
+    """bench.py --dump-outputs: float32 / float64 arrays only, at most 64 MB, and for a batch larger than DUMP_MAX_RAYS the
+    same seeded sample every time, each record next to the index of its ray."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    from bvh_b200.api import HIT3F
+    n = bench.DUMP_MAX_RAYS + 4321
+    rec = np.zeros(n, HIT3F)
+    rec["prim_id"] = np.arange(n)
+    rec["prim_id"][::7] = 0xFFFFFFFF
+    rec["t"], rec["u"], rec["v"] = np.arange(n) * 0.5, np.arange(n) * 0.25, np.arange(n) * 0.125
+    hits = torch.from_numpy(rec.view(np.int32).reshape(n, 4))
+    for out in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / out), hits, HIT3F)
+    total = 0
+    got = {}
+    for name in ("prim_id", "t", "u", "v", "ray_index"):
+        a, b = np.load(tmp_path / "a" / f"{name}.npy"), np.load(tmp_path / "b" / f"{name}.npy")
+        assert a.dtype in (np.float32, np.float64) and a.shape == (bench.DUMP_MAX_RAYS,) and np.array_equal(a, b)
+        total += a.nbytes
+        got[name] = a
+    assert total <= 64 << 20
+    index = got["ray_index"].astype(np.int64)
+    assert (np.diff(index) > 0).all() and index[-1] < n
+    assert np.array_equal(got["prim_id"], rec["prim_id"][index].astype(np.float64))
+    assert (got["prim_id"][index % 7 == 0] == 0xFFFFFFFF).all()
+    for name in ("t", "u", "v"):
+        assert np.array_equal(got[name], rec[name][index])

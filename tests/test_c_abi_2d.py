@@ -1,18 +1,20 @@
 """2-D suffixes of the C ABI (bvh2f / bvh2d, reference c_api/bvh.cpp:7-25).
 
-CPU part: a tree built and saved by the UNMODIFIED reference C library (oracle/_ref/libbvh_c_ref.so) is
-loaded through our library; node accessors, per-ray callback traversal (all four variants), refit and save
-must then agree with the reference bit for bit.  GPU part: bvh2f_build / bvh2d_build (the LBVH pipeline on
-boxes lifted to z = 0) produce a valid tree whose traversal finds the brute-force answer."""
+CPU part: the file of a tree built and saved by the UNMODIFIED reference C library (rebuilt from its stored topology,
+tests/golden/make_ref_digests.py) is loaded through our library; node accessors, per-ray callback traversal (all four
+variants), refit and save must then agree with the reference's stored answers bit for bit.  GPU part: bvh2f_build /
+bvh2d_build (the LBVH pipeline on boxes lifted to z = 0) produce a valid tree whose traversal finds the brute-force
+answer."""
 import ctypes as C
 import os
 
 import numpy as np
 import pytest
 
+from tests.helpers import digest, ref_digests, tree_blob
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OURS = os.path.join(ROOT, "bvh_b200", "libbvh_c.so")
-REF = os.path.join(ROOT, "oracle", "_ref", "libbvh_c_ref.so")
 libc = C.CDLL(None)
 libc.fopen.restype = C.c_void_p
 libc.fopen.argtypes = [C.c_char_p, C.c_char_p]
@@ -127,40 +129,41 @@ def scene2(n, seed, dtype):
     return boxes, centers, rays
 
 
-needs_ref = pytest.mark.skipif(not os.path.exists(REF), reason="oracle/_ref not built")
-
-
-@needs_ref
 @pytest.mark.parametrize("s", ["2f", "2d"])
 def test_loaded_reference_tree_behaves_like_the_reference(tmp_path, s):
-    ours, ref = Api2(OURS, s), Api2(REF, s)
+    ours = Api2(OURS, s)
+    want = ref_digests(f"c_abi_2d/{s}")
     boxes, centers, rays = scene2(700, 3, ours.dtype)
-    rb = ref.build(boxes, centers)
+    with np.load(os.path.join(ROOT, "tests", "golden", "ref_topology.npz")) as g:
+        stored = {k[len(f"c_abi_2d/{s}/"):]: g[k] for k in g.files if k.startswith(f"c_abi_2d/{s}/")}
+    blob = tree_blob(stored["index"], stored["prim_ids"], boxes, 2)
+    assert digest(blob) == want["blob"]
     path = str(tmp_path / f"tree_{s}.bin")
-    ref.save(rb, path)
+    open(path, "wb").write(blob)
     ob = ours.load(path)
-    assert ours.f("get_node_count")(ob) == ref.f("get_node_count")(rb) > 1
-    assert ours.nodes(ob) == ref.nodes(rb)
-    ids = ref.prim_ids(rb)
+    assert ours.f("get_node_count")(ob) == stored["index"].shape[0] > 1
+    assert digest(np.array(ours.nodes(ob), np.float64)) == want["nodes"]
+    ids = [int(i) for i in stored["prim_ids"]]
     assert ours.prim_ids(ob) == ids and sorted(ids) == list(range(700))
     for variant in ("intersect_ray", "intersect_ray_any", "intersect_ray_robust", "intersect_ray_any_robust"):
-        got, want = ours.trace(ob, rays, boxes, ids, variant), ref.trace(rb, rays, boxes, ids, variant)
-        assert got == want, variant                        # same hits AND the same sequence of leaf visits
+        got = ours.trace(ob, rays, boxes, ids, variant)
+        ref = [(int(i), None if np.isnan(t) else float(t), int(c))
+               for i, t, c in zip(*(stored[f"{variant}/{k}"] for k in ("id", "t", "calls")))]
+        assert got == ref, variant                         # same hits AND the same sequence of leaf visits
         assert sum(1 for g in got if g[0] >= 0) > 50
 
     # grow every leaf box, refit, and compare again; then save and compare the bytes
-    for api, bvh in ((ours, ob), (ref, rb)):
-        for i in range(api.f("get_node_count")(bvh)):
-            nd = api.f("get_node")(bvh, i)
-            if api.g("is_leaf")(nd):
-                b = api.g("get_bbox")(nd)
-                b.max.x += 0.25; b.min.y -= 0.125
-                api.g("set_bbox")(nd, C.byref(b))
-        api.f("refit")(bvh)
-    assert ours.nodes(ob) == ref.nodes(rb)
-    p1, p2 = str(tmp_path / "a.bin"), str(tmp_path / "b.bin")
-    ours.save(ob, p1); ref.save(rb, p2)
-    assert open(p1, "rb").read() == open(p2, "rb").read()
+    for i in range(ours.f("get_node_count")(ob)):
+        nd = ours.f("get_node")(ob, i)
+        if ours.g("is_leaf")(nd):
+            b = ours.g("get_bbox")(nd)
+            b.max.x += 0.25; b.min.y -= 0.125
+            ours.g("set_bbox")(nd, C.byref(b))
+    ours.f("refit")(ob)
+    assert digest(np.array(ours.nodes(ob), np.float64)) == want["refit_nodes"]
+    p1 = str(tmp_path / "a.bin")
+    ours.save(ob, p1)
+    assert digest(open(p1, "rb").read()) == want["refit_blob"]
 
     # node editing entry points
     nd = ours.f("get_node")(ob, 1)
@@ -169,7 +172,7 @@ def test_loaded_reference_tree_behaves_like_the_reference(tmp_path, s):
     count = ours.f("get_node_count")(ob)
     ours.f("append_node")(ob); assert ours.f("get_node_count")(ob) == count + 1
     ours.f("remove_last_node")(ob); assert ours.f("get_node_count")(ob) == count
-    ours.f("destroy")(ob); ref.f("destroy")(rb)
+    ours.f("destroy")(ob)
 
 
 @pytest.mark.gpu

@@ -1,24 +1,24 @@
 """bvhNN_optimize / bvh_optimize_nodes = the reference's ReinsertionOptimizer (reinsertion_optimizer.h:27-30,88-267).
 
-A tree built by the UNMODIFIED reference C library (oracle/_ref/libbvh_c_ref.so) is optimised twice: by the
-reference's own bvhNN_optimize and by this library (bvh_optimize_nodes on the same node array, and — for the 2-D
-suffixes, which need no GPU — bvh2f_load + bvh2f_optimize + bvh2f_save).  The results must be identical node for
-node, serial and multi-threaded, and the pass must actually lower the tree's SAH cost."""
+A tree built by the UNMODIFIED reference C library is optimised twice: by the reference's own bvhNN_optimize and by this
+library (bvh_optimize_nodes on the same node array, and — for the 2-D suffixes, which need no GPU — bvh2f_load +
+bvh2f_optimize + bvh2f_save).  The results must be identical node for node, serial and multi-threaded, and the pass must
+actually lower the tree's SAH cost.  The reference's side is stored (tests/golden/make_ref_digests.py): the topology of
+the tree it builds, from which tests/helpers.py tree_blob rebuilds its exact file, and digests of what its pass returns."""
 import ctypes as C
 import os
 
 import numpy as np
 import pytest
 
+from tests.helpers import digest, ref_digests, tree_blob
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OURS = os.path.join(ROOT, "bvh_b200", "libbvh_c.so")
-REF = os.path.join(ROOT, "oracle", "_ref", "libbvh_c_ref.so")
 libc = C.CDLL(None)
 libc.fopen.restype = C.c_void_p
 libc.fopen.argtypes = [C.c_char_p, C.c_char_p]
 libc.fclose.argtypes = [C.c_void_p]
-
-pytestmark = pytest.mark.skipif(not os.path.exists(REF), reason="oracle/_ref (the compiled reference) is not available")
 
 
 def bind(lib, s):
@@ -33,10 +33,6 @@ def bind(lib, s):
     lib.bvh_thread_pool_create.argtypes = [C.c_size_t]
     lib.bvh_thread_pool_destroy.argtypes = [C.c_void_p]
     return f
-
-
-class Config(C.Structure):
-    _fields_ = [("quality", C.c_int), ("min_leaf_size", C.c_size_t), ("max_leaf_size", C.c_size_t), ("parallel_threshold", C.c_size_t)]
 
 
 def save_bytes(f, bvh, path):
@@ -81,33 +77,28 @@ def scene(dim, n, dtype, seed):
 @pytest.mark.parametrize("s,dim,dtype", [("3f", 3, np.float32), ("3d", 3, np.float64), ("2f", 2, np.float32), ("2d", 2, np.float64)])
 @pytest.mark.parametrize("n", [300, 3000])
 def test_optimize_nodes_equals_the_reference(tmp_path, s, dim, dtype, n):
-    ref, ours = C.CDLL(REF), C.CDLL(OURS)
-    rf = bind(ref, s)
+    ours = C.CDLL(OURS)
     boxes, centers = scene(dim, n, dtype, 7 + n)
-    cfg = Config(1, 1, 8, 1024)                                   # Quality::Medium: SweepSAH without the optimizer
-    tree = rf("build")(None, boxes.ctypes.data, centers.ctypes.data, n, C.byref(cfg))
-    before = save_bytes(rf, tree, tmp_path / "before.bin")
-    pool = ref.bvh_thread_pool_create(4)
-    rf("optimize")(pool if n > 100 else None, tree)
-    ref.bvh_thread_pool_destroy(pool)
-    after_ref = save_bytes(rf, tree, tmp_path / "after_ref.bin")
-    rf("destroy")(tree)
+    ref = ref_digests(f"optimize/{s}/{n}")
+    with np.load(os.path.join(ROOT, "tests", "golden", "ref_topology.npz")) as g:
+        before = tree_blob(g[f"optimize/{s}/{n}/index"], g[f"optimize/{s}/{n}/prim_ids"], boxes, dim)
+    assert digest(before) == ref["before"], "the stored topology no longer gives the reference's tree"
     if n >= 3000:
-        assert after_ref != before, "the scene must give the optimizer something to do"
+        assert ref["after"] != ref["before"], "the scene must give the optimizer something to do"
+    (tmp_path / "before.bin").write_bytes(before)
 
     nodes, ids = parse(before, dim, dtype)
-    want, want_ids = parse(after_ref, dim, dtype)
-    assert sah_cost(want, dim) <= sah_cost(nodes, dim)
-    if n >= 3000:
-        assert sah_cost(want, dim) < sah_cost(nodes, dim)
     ours.bvh_optimize_nodes.argtypes = [C.c_void_p, C.c_size_t, C.c_int, C.c_int, C.c_double, C.c_size_t, C.c_size_t]
     ours.bvh_last_error.restype = C.c_char_p
     for threads in (1, 5):
         mine = nodes.copy()
         rc = ours.bvh_optimize_nodes(mine.ctypes.data, mine.shape[0], dim, dtype == np.float64, 0.05, 3, threads)
         assert rc == 0, ours.bvh_last_error()
-        assert mine.tobytes() == want.tobytes(), f"{threads} thread(s): tree differs from the reference's optimised tree"
-    assert np.array_equal(ids, want_ids)                          # the pass never touches the primitive order
+        assert digest(mine) == ref["after_nodes"], f"{threads} thread(s): tree differs from the reference's optimised tree"
+    assert digest(ids) == ref["after_prim_ids"]                   # the pass never touches the primitive order
+    assert sah_cost(mine, dim) <= sah_cost(nodes, dim)            # `mine` is now bit for bit the reference's result
+    if n >= 3000:
+        assert sah_cost(mine, dim) < sah_cost(nodes, dim)
 
     if dim == 2:                                                  # the host-only suffixes: through load / optimize / save
         of = bind(ours, s)
@@ -115,7 +106,7 @@ def test_optimize_nodes_equals_the_reference(tmp_path, s, dim, dtype, n):
         opool = ours.bvh_thread_pool_create(3)
         of("optimize")(opool, h)
         ours.bvh_thread_pool_destroy(opool)
-        assert save_bytes(of, h, tmp_path / "after_ours.bin") == after_ref
+        assert digest(save_bytes(of, h, tmp_path / "after_ours.bin")) == ref["after"]
         of("destroy")(h)
 
 

@@ -1,14 +1,14 @@
 """Pins the plain-C oracle (oracle/bvh_oracle.c) to the reference:
   (1) the reference's own known answers (SURVEY.md §4 / BASELINE.md §2), via committed golden files
       produced by tests/golden/make_golden.py from the unmodified reference;
-  (2) the unmodified reference itself (oracle/_ref), when it was built here.
+  (2) the unmodified reference's outputs on seeded scenes, stored as SHA-256 digests by tests/golden/make_ref_digests.py.
 Everything is bit-exact: node arrays, prim ids, hit ids, t, u, v and the per-ray step counters."""
 import numpy as np
 import pytest
 
 from oracle.pyoracle import ANY_HIT, ROBUST, TIE_LOWEST_ID
 from tests.conftest import golden
-from tests.helpers import assert_hits_equal
+from tests.helpers import assert_hits_equal, digest, ref_digests
 
 MODES = (("lowest", TIE_LOWEST_ID), ("last", 0), ("any", ANY_HIT | TIE_LOWEST_ID), ("robust", ROBUST | TIE_LOWEST_ID))
 
@@ -78,55 +78,54 @@ def test_golden_scenes(oracle, name):
 
 @pytest.mark.parametrize("kind,n,dtype", [("soup", 3000, np.float32), ("grid", 3000, np.float32), ("soup", 1500, np.float64)])
 @pytest.mark.parametrize("quality", ["low", "medium"])
-def test_builders_match_reference(oracle, ref, kind, n, dtype, quality):
+def test_builders_match_reference(oracle, kind, n, dtype, quality):
     """The restated BinnedSah / SweepSah builders give the reference's exact node array and prim ids
     (serial DefaultBuilder overload, default_builder.h:49-62)."""
     from bvh_b200 import scenes
+    want = ref_digests(f"builders/{kind}-{n}-{np.dtype(dtype).name}/{quality}")
     tris = scenes.make_mesh(kind, n, dtype=dtype)
     bo, co = oracle.tri_bboxes_centers(tris)
-    br, cr = ref.tri_bboxes_centers(tris)
-    assert (bo == br).all() and (co == cr).all()
+    assert digest(bo) == want["bboxes"] and digest(co) == want["centers"]
     to = oracle.build(bo, co, quality=quality)
-    tr = ref.build(br, cr, quality=quality, threads=-1)
-    ao, ar = to.arrays(), tr.arrays()
-    assert ao[0].shape == ar[0].shape and (ao[0] == ar[0]).all() and (ao[1] == ar[1]).all() and (ao[2] == ar[2]).all()
+    for name, a in zip(("bounds", "index", "prim_ids"), to.arrays()):
+        assert digest(a) == want[name], f"{kind}/{quality}: {name} differs from the reference's"
     assert oracle.check_invariants(to, 8) == 0
-    assert oracle.serialize(to) == ref.serialize(tr)
+    assert digest(oracle.serialize(to)) == want["serialized"]
     oracle.set_triangles(to, tris)
-    ref.set_triangles(tr, tris)
     rays = scenes.make_primary(kind, 96, 96, dtype=dtype)
-    for _, flags in MODES:
+    for mode, flags in MODES:
         a = oracle.trace(to, rays, flags=flags, stats=True)
-        b = ref.trace(tr, rays, flags=flags, stats=True)
-        assert_hits_equal(a[:4], b[:4], f"{kind}/{quality}/{flags}")
-        assert (a[4] == b[4]).all()
+        for name, got in zip(("ids", "t", "u", "v", "stats"), a):
+            assert digest(got) == want[f"{mode}_{name}"], f"{kind}/{quality}/{mode}: {name} differs from the reference's"
 
 
-def test_refit_matches_reference(oracle, ref):
+def test_refit_matches_reference(oracle):
     from bvh_b200 import scenes
+    want = ref_digests("refit")
     tris = scenes.soup(2000)
-    bb, cc = ref.tri_bboxes_centers(tris)
-    tr = ref.build(bb, cc, quality="medium", threads=-1)
-    bounds, idx, ids = tr.arrays()
+    bb, cc = oracle.tri_bboxes_centers(tris)
+    bounds, idx, ids = oracle.build(bb, cc, quality="medium").arrays()        # the reference's tree (pinned above)
+    assert digest(bounds) == want["bounds"] and digest(idx) == want["index"] and digest(ids) == want["prim_ids"]
     rng = np.random.RandomState(3)
     leaf = (idx & 15) != 0
     noisy = bounds.copy()
     noisy[leaf] += rng.uniform(-0.01, 0.01, size=noisy[leaf].shape).astype(np.float32)
     noisy[~leaf] = 0
     a = oracle.from_arrays(noisy, idx, ids)
-    b = ref.from_arrays(noisy, idx, ids)
     oracle.refit(a)
-    ref.refit(b)
-    assert (a.arrays()[0] == b.arrays()[0]).all()
+    assert digest(a.arrays()[0]) == want["refitted"]
 
 
-def test_morton_matches_reference(oracle, ref):
+def test_morton_matches_reference(oracle):
     rng = np.random.RandomState(7)
+    m32, m64 = [], []
     for _ in range(500):
         x, y, z = (int(v) for v in rng.randint(0, 1 << 10, 3))
-        assert oracle.morton_encode(x, y, z, 32) == ref.morton_encode(x, y, z, 32)
+        m32.append(oracle.morton_encode(x, y, z, 32))
         x, y, z = (int(v) for v in rng.randint(0, 1 << 21, 3))
-        assert oracle.morton_encode(x, y, z, 64) == ref.morton_encode(x, y, z, 64)
+        m64.append(oracle.morton_encode(x, y, z, 64))
+    want = ref_digests("morton")
+    assert digest(np.array(m32, np.uint32)) == want["code32"] and digest(np.array(m64, np.uint64)) == want["code64"]
 
 
 def test_fma_configuration(oracle):
